@@ -10,7 +10,7 @@ import tvm_b200
 from oracle import tracegen as tg
 
 import test_vm_programs as tvp
-from test_main_fill_host import _program, _ev
+from test_main_fill_host import _program, _ev, host  # noqa: F401 - `host` is the fixture that builds the host harness
 
 pytestmark = pytest.mark.gpu
 P = tg.P
@@ -96,23 +96,19 @@ def test_plain_c_aet_client_proves_halt_on_the_gpu(tmp_path):
 
 
 @pytest.mark.parametrize("k", [13, 16, 18])
-def test_device_fill_equals_the_host_executor_on_a_synthetic_aet(backend, k):
+def test_device_fill_equals_the_host_executor_on_a_synthetic_aet(backend, host, k):
     """Sizes no program of the test suite reaches (2^16 rows: 2^15 RAM rows over 2^14 unique pointers -> subproduct tree of 14
     levels with the transform paths, radix sorts of 2^16 keys, 44 000 u32 rows): the CUDA executor against the sequential
     host executor running the same stage bodies (tests/host/main_fill_host.cu, itself checked against the oracle on real
     programs by tests/test_main_fill_host.py)."""
-    import ctypes
-    import importlib.util
     import os
-    from test_main_fill_host import SO, host_main_table
-    if not os.path.exists(SO):
-        pytest.skip("host harness not built (tests/test_main_fill_host.py builds it where nvcc is available)")
+    from test_main_fill_host import host_main_table
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     src = open(os.path.join(root, "tools", "fill_time.py")).read().split("b = tvm_b200.Backend(0)")[0]
     ns = {"__file__": os.path.join(root, "tools", "fill_time.py")}
     exec(compile(src, "fill_time", "exec"), ns)
     aet = ns["synthetic_aet"](k, np.random.default_rng(k))
-    want, want_lengths = host_main_table(ctypes.CDLL(SO), aet, 1 << k)
+    want, want_lengths = host_main_table(host, aet, 1 << k)
     got, lengths = backend.main_table_from_aet(aet, 1 << k)
     assert lengths == want_lengths
     bad = [c for c in range(149) if not np.array_equal(got[c], want[c])]
